@@ -285,6 +285,51 @@ def parity_check_multi(engine, group, rank, world, dev, lr=1e-3):
     return res
 
 
+DUMP_ROWS_PER_GROUP = 4096
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, engine, group, ids, seed=0):
+    """Writes what the last timed step computed as float32 / float64 .npy files under out_dir, so that two builds
+    run with the same arguments (hence the same inputs) can be compared array by array:
+      loss [1], logits [B] (fused towers only)   what the step returned / wrote for its batch
+      dense_params [n]                           the tower parameters the PS holds after the step, flat order
+      row_ids [K, 2] float64                     (id group, id): a fixed seeded sample of up to DUMP_ROWS_PER_GROUP
+                                                 of the distinct ids of the step's batch in every group
+      deep_rows [K, 8], wide_rows [K]            those rows of the deep / wide tables after the step
+    Gradients are summed with atomics, so repeated runs of one build differ in the last bits: compare with a float
+    tolerance (two runs at the defaults on a B200 at its 1000 W power limit: rows and dense parameters within 6e-8,
+    logits within 6e-7).
+    ids: the step's int64 [G, B] id batch (device)."""
+    import numpy as np
+    import torch
+
+    torch.cuda.synchronize(engine.device)
+    out = {"loss": engine.loss_buf.cpu().numpy().astype(np.float32)}
+    if engine.tower_kind != "torch":  # the torch tower returns its logits to autograd, not into logits_buf
+        out["logits"] = engine.logits_buf.cpu().numpy().astype(np.float32)
+    dense = group.pull_dense([n for n, _ in engine.params])
+    out["dense_params"] = torch.cat([dense[n].reshape(-1) for n, _ in engine.params]).cpu().numpy()
+    picks, requests = [], []
+    for g in range(engine.G):
+        u = torch.unique(ids[g]).cpu().numpy()
+        rng = np.random.RandomState(seed + g)
+        sel = u[np.sort(rng.choice(u.size, min(u.size, DUMP_ROWS_PER_GROUP), replace=False))]
+        picks.append(np.stack([np.full(sel.size, g), sel], 1).astype(np.float64))
+        requests += [(engine.deep_names[g], sel), (engine.wide_names[g], sel)]
+    rows = group.pull_rows(requests)
+    out["row_ids"] = np.concatenate(picks)
+    out["deep_rows"] = torch.cat(rows[0::2]).cpu().numpy()
+    out["wide_rows"] = torch.cat(rows[1::2]).reshape(-1).cpu().numpy()
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("bench.py --dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def api_path_leg(dev, batches, steps, warmup):
     """The same DeepFM step through the DROP-IN API instead of the engine: ParameterServerTrainer.train_minibatch
     over 76 elasticdl Embedding layers + PSClient (worker/ps_trainer.py), tower in eager torch.  Timed by wall
@@ -363,6 +408,9 @@ def main():
     ap.add_argument("--no-parity-check", action="store_true", help="skip the post-timing N>1 parity self-check")
     ap.add_argument("--ids", default="narrow", choices=["narrow", "int32"],
                     help="id transport of the packed batches: 1/2/4 bytes per id by table size, or int32")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (loss, logits, dense "
+                         "parameters, a fixed seeded sample of the embedding rows it trained) as DIR/<name>.npy")
     args = ap.parse_args()
     cpu_batch = args.cpu_batch or args.batch
 
@@ -520,6 +568,11 @@ def main():
         ms = max_over_ranks(e0.elapsed_time(e1))
         group.check()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # step i of a timed loop trains batch i % pool: the graph loop ran steps warmup .. warmup+steps-1, the
+        # eager path's last loop steps 0 .. steps-1
+        last = (args.warmup + args.steps - 1 if use_graph else args.steps - 1) % args.pool
+        dump_outputs(args.dump_outputs, engine, group, devb[last][0])
 
     # ---- per-kernel durations from the CUDA events recorded inside the timed region ----
     kern = engine.kernel_report(ev, [uniq_per_batch[i % args.pool] for i in range(args.steps)])
